@@ -1,19 +1,16 @@
 #!/usr/bin/env python
-"""Converter: the reference checkout's operator fixtures -> one pickle-free .npz next to this package.
+"""Converter: the reference checkout's operator fixtures -> the pickle-free tests/golden/smpl_topology.*.npz.
 
 The reference ships its fixed mesh hierarchy as pickled scipy CSC matrices
 (<CAPE checkout>/data/transform_matrices/{for_demo,ds2}/{A,D,U}.npy, loaded at lib/load_data.py:7-32 with
-encoding='latin1').  Those files are covered by the reference's licence (no redistribution), so this repository
-does NOT contain them or anything derived loss-free from them: the .npz is generated locally from the user's own
-checkout of qianlim/CAPE and is git-ignored.  It holds the operators as plain CSR arrays
+encoding='latin1').  The files written here are the copy `cape_b200.topology` reads; they come from the reference's
+data/ directory and fall under the reference's licence.  They hold the operators as plain CSR arrays
 (indptr/indices/data/shape), the SMPL edge table (data/edges_smpl.npy, used by lib/losses.py:9-25; = upper triangle
 of A[0], checked against the reference file), the per-vertex normalisation statistics
 (data/demo_data/trainset_stats.npz, demos.py:155), the clothing-vertex index list, the template mesh and the demo
-poses (demos.py:349-357).
+poses (demos.py:349-357), split in the parts of `topology.DATA_PARTS` (each well under 1 MB).
 
-    python -m cape_b200.pack_topology [--reference /path/to/CAPE]        (default: $CAPE_REFERENCE, /root/reference)
-
-`__graft_entry__.build()` runs it when the file is missing; `cape_b200.topology` does so on first use.
+    python -m cape_b200.pack_topology --reference /path/to/CAPE        (default: $CAPE_REFERENCE)
 """
 import argparse
 import os
@@ -21,18 +18,10 @@ import sys
 import numpy as np
 import scipy.sparse as sp
 
-OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "data", "smpl_topology.npz")
+from cape_b200 import topology
 
 
-def default_reference():
-    """The reference checkout to read the fixtures from: $CAPE_REFERENCE, else /root/reference; None if absent."""
-    for cand in (os.environ.get("CAPE_REFERENCE"), "/root/reference"):
-        if cand and os.path.isdir(os.path.join(cand, "data", "transform_matrices")):
-            return cand
-    return None
-
-
-def pack(REF, OUT=OUT):
+def pack(REF, out_dir=topology.DATA_DIR):
     def _load(kind, name):
         path = os.path.join(REF, "data", "transform_matrices", kind, name + ".npy")
         return list(np.load(path, encoding="latin1", allow_pickle=True))
@@ -72,22 +61,23 @@ def pack(REF, OUT=OUT):
     out["template.v"], out["template.f"] = np.asarray(v, np.float64), np.asarray(f, np.int32)
     dp = np.load(os.path.join(REF, "data", "demo_data", "demo_pose_params.npz"))
     out["demo.rot"], out["demo.pose"] = dp["rot"], dp["pose"]
-    os.makedirs(os.path.dirname(OUT), exist_ok=True)
-    tmp = OUT + ".tmp.%d.npz" % os.getpid()
-    np.savez_compressed(tmp, **out)
-    os.replace(tmp, OUT)                     # atomic: concurrent ranks may all find the file missing
-    return OUT
+    os.makedirs(out_dir, exist_ok=True)
+    part_of = lambda key: key.split(".")[0] if key.split(".")[0] in ("for_demo", "ds2") else "assets"
+    files = topology.data_files(out_dir)
+    for part, fn in zip(topology.DATA_PARTS, files):
+        np.savez_compressed(fn, **{k: v for k, v in out.items() if part_of(k) == part})
+    return files
 
 
 def main(argv=None):
     ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
-    ap.add_argument("--reference", default=default_reference(), help="checkout of qianlim/CAPE")
-    ap.add_argument("--out", default=OUT)
+    ap.add_argument("--reference", default=os.environ.get("CAPE_REFERENCE"), help="checkout of qianlim/CAPE")
+    ap.add_argument("--out-dir", default=topology.DATA_DIR)
     a = ap.parse_args(argv)
     if not a.reference:
-        ap.error("no reference checkout found: pass --reference or set CAPE_REFERENCE")
-    out = pack(a.reference, a.out)
-    print("wrote", os.path.abspath(out), os.path.getsize(out), "bytes")
+        ap.error("no reference checkout given: pass --reference or set CAPE_REFERENCE")
+    for fn in pack(a.reference, a.out_dir):
+        print("wrote", os.path.abspath(fn), os.path.getsize(fn), "bytes")
 
 
 if __name__ == "__main__":

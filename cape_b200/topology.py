@@ -3,8 +3,8 @@
 Host-side counterpart of the reference's topology prep:
   - `laplacian`, `rescale_L`  : lib/mesh_sampling.py:10-38 (same names, same arithmetic in fp32)
   - `load_graph_mtx`          : lib/load_data.py:7-32 (same return convention) -- reads the pickle-free
-                                copy of data/transform_matrices/** that cape_b200/pack_topology.py makes
-                                from the user's reference checkout (licensed data: not part of this repo)
+                                copy of data/transform_matrices/** under tests/golden/ (made by
+                                cape_b200/pack_topology.py from a checkout of the reference)
 The reference turns every scipy matrix into a tf.SparseTensor and runs one SpMM per Chebyshev order and
 per pool/unpool (lib/models.py:74-96,141-149).  Here the operators are constants, so they are composed
 offline:  op_k = D . T_k(L~) . U  -- one sparse "row-gather" per polynomial order with pooling (row
@@ -15,8 +15,14 @@ import os
 import numpy as np
 import scipy.sparse as sp
 
-_DATA = os.path.join(os.path.dirname(os.path.abspath(__file__)), "data", "smpl_topology.npz")
+DATA_DIR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+# the fixtures are split in parts so that no single file grows past 1 MB
+DATA_PARTS = ("for_demo", "ds2", "assets")
 _cache = {}
+
+
+def data_files(directory=DATA_DIR):
+    return [os.path.join(directory, "smpl_topology.%s.npz" % part) for part in DATA_PARTS]
 
 
 def laplacian(W, normalized=True):
@@ -43,16 +49,11 @@ def rescale_L(L, lmax=2):
 
 def _npz():
     if "npz" not in _cache:
-        if not os.path.exists(_DATA):
-            from . import pack_topology
-            ref = pack_topology.default_reference()
-            if ref is None:
-                raise FileNotFoundError(
-                    "%s missing and no reference checkout to build it from: the SMPL mesh hierarchy is licensed data of "
-                    "qianlim/CAPE and is not shipped here.  Run `python -m cape_b200.pack_topology --reference "
-                    "/path/to/CAPE` (or set CAPE_REFERENCE) once." % _DATA)
-            pack_topology.pack(ref, _DATA)
-        _cache["npz"] = np.load(_DATA)
+        z = {}
+        for fn in data_files():
+            with np.load(fn) as part:
+                z.update((k, part[k]) for k in part.files)
+        _cache["npz"] = z
     return _cache["npz"]
 
 
@@ -69,7 +70,7 @@ def _mats(kind, name, dtype):
 def load_graph_mtx(project_dir=None, load_for_demo=False):
     """Same contract as lib/load_data.py:7-32: returns L_ds2, D_ds2, U_ds2 or, with load_for_demo,
     L, D, U, p, L_ds2, D_ds2, U_ds2 (all fp32; L = normalised Laplacians of the adjacency fixtures).
-    `project_dir` is accepted for signature compatibility and ignored (fixtures live inside the package)."""
+    `project_dir` is accepted for signature compatibility and ignored (the fixtures are read from DATA_DIR)."""
     A_ds2, D_ds2, U_ds2 = (_mats("ds2", n, np.float32) for n in "ADU")
     L_ds2 = [laplacian(a, normalized=True) for a in A_ds2]
     if not load_for_demo:
@@ -97,16 +98,12 @@ def clothing_verts_idx():
 def template_mesh():
     """(vertices [6890, 3] float64, faces [13776, 3] int32) of data/template_mesh.obj (demos.py:352-353)."""
     z = _npz()
-    if "template.v" not in z.files:
-        raise FileNotFoundError("%s predates the demo assets: delete it and re-run cape_b200.pack_topology" % _DATA)
     return z["template.v"], z["template.f"]
 
 
 def demo_pose_params():
     """(rot [6, 216], pose [6, 72]) of data/demo_data/demo_pose_params.npz (demos.py:355-356)."""
     z = _npz()
-    if "demo.rot" not in z.files:
-        raise FileNotFoundError("%s predates the demo assets: delete it and re-run cape_b200.pack_topology" % _DATA)
     return z["demo.rot"], z["demo.pose"]
 
 

@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Golden vectors from the REFERENCE's own model code.  Runs only where /root/reference (or $CAPE_REFERENCE) exists.
+"""Golden vectors from the REFERENCE's own model code.  Runs only where $CAPE_REFERENCE names its checkout.
 
 `lib/models.py` of the reference is imported UNMODIFIED and executed on the TensorFlow-1 API shim of
 oracle/tf1_shim.py (torch-CPU behind the ~70 TF symbols the file calls): `CAPE.build_graph(phase='train')` then runs
@@ -21,7 +21,7 @@ Inputs are the ones tests/parity.train_step uses (batch of 2 from cape_b200.synt
 calibrated initial parameters, global_step 100), so the GPU parity tests, the oracle and this file meet on one update.
 A second, smaller run covers the non-affine (GroupNorm) decoder of configs/CAPE_nz18_*.yaml at batch 1.
 
-    python tests/golden/make_ref_golden.py          (about a minute)
+    CAPE_REFERENCE=/path/to/CAPE python tests/golden/make_ref_golden.py          (about a minute)
 """
 import os
 import sys
@@ -31,11 +31,11 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.abspath(os.path.join(HERE, "..", ".."))
-REF = os.environ.get("CAPE_REFERENCE", "/root/reference")
+REF = os.environ.get("CAPE_REFERENCE", "")
 for p in (ROOT, os.path.join(ROOT, "tests")):
     if p not in sys.path:
         sys.path.insert(0, p)
-if REF not in sys.path:
+if REF and REF not in sys.path:
     sys.path.append(REF)            # last: only `lib` (the reference's package) is meant to resolve there
 
 OUT = os.path.join(HERE, "ref_models_golden.npz")

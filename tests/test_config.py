@@ -1,11 +1,20 @@
-"""parse_config: reference flags/defaults/precedence; the reference's own yaml files load unchanged."""
+"""parse_config: reference flags/defaults/precedence; the reference's own yaml files load unchanged.
+
+The reference's yaml files and the flag table of its own parse_config are recorded in
+tests/golden/ref_config_golden.json (tests/golden/make_ref_host_golden.py)."""
+import json
 import os
 
 import pytest
 
 from cape_b200.config_parser import model_params, parse_config
 
-REF_CFG = "/root/reference/configs"
+REF_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_config_golden.json")
+
+
+def _ref_golden():
+    with open(REF_GOLDEN) as f:
+        return json.load(f)
 
 AFFINE_YAML = """dataset: dataset_male_4clotypes
 name: CAPE-affineconv_nz64_pose32_clotype32_male
@@ -56,10 +65,12 @@ def test_defaults_without_file(tmp_path, monkeypatch):
         parse_config(["--config", "missing.yaml"])
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CFG), reason="reference tree not present (GPU box)")
-def test_reference_configs_load_unchanged():
-    for fn in sorted(os.listdir(REF_CFG)):
-        args, _ = parse_config(["--config", os.path.join(REF_CFG, fn)])
+def test_reference_configs_load_unchanged(tmp_path):
+    configs = _ref_golden()["configs"]
+    assert len(configs) == 8
+    for fn, text in sorted(configs.items()):
+        (tmp_path / fn).write_text(text)
+        args, _ = parse_config(["--config", str(tmp_path / fn)])
         if fn.startswith("CAPE-affineconv_nz64"):
             assert (args.nz, args.nz_cond, args.nz_cond2, args.affine) == (64, 32, 32, 1)
         if fn.startswith("CAPE_nz18"):
@@ -133,42 +144,21 @@ def test_layer_forms_of_the_shipped_config():
     assert f(512, 64, 256, 2, 862, 862, True, True, "gside", False, False, "dec/aff1", {"CAPE_FWD_MODE": "basis"})[0] == "fused"
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CFG), reason="reference tree not present (GPU box)")
-def test_flag_inventory_is_the_references(monkeypatch):
+def test_flag_inventory_is_the_references():
     """Every flag the reference's own parse_config declares (config_parser.py:11-63) -- name, type, default, choices --
-    against the table this package parses with.  The reference needs `configargparse` (not installed): a recording
-    stand-in captures its add_argument calls while its unmodified parse_config runs."""
-    import argparse
-    import importlib.util
-    import sys
-    import types
+    against the table this package parses with.  The reference needs `configargparse` (not installed): its table was
+    recorded by a stand-in that captured its add_argument calls while its unmodified parse_config ran."""
     from cape_b200 import config_parser as ours
-    recorded = []
-
-    class ArgParser(object):
-        def __init__(self, *a, **k):
-            pass
-
-        def add_argument(self, flag, **kw):
-            recorded.append((flag.lstrip("-"), kw))
-
-        def parse_known_args(self, *a, **k):
-            return argparse.Namespace(**{n: kw.get("default") for n, kw in recorded}), []
-
-    stub = types.ModuleType("configargparse")
-    stub.ArgParser, stub.ArgumentDefaultsHelpFormatter, stub.DefaultConfigFileParser = ArgParser, object, object
-    monkeypatch.setitem(sys.modules, "configargparse", stub)
-    spec = importlib.util.spec_from_file_location("ref_config_parser", os.path.join(os.path.dirname(REF_CFG), "config_parser.py"))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    args, args_dict = mod.parse_config()
-    assert recorded[0][0] == "config" and recorded[0][1]["is_config_file"] and recorded[0][1]["default"] == ours.DEFAULT_CONFIG
-    ref = [(n, kw.get("type", str), kw.get("default"), kw.get("choices")) for n, kw in recorded[1:]]
-    mine = [(n, t, d, ours._CHOICES.get(n)) for n, t, d, _ in ours._SPEC]
+    g = _ref_golden()
+    cf = g["config_flag"]
+    assert cf["name"] == "config" and cf["is_config_file"] and cf["default"] == ours.DEFAULT_CONFIG
+    ref = [tuple(r) for r in g["flags"]]
+    mine = [(n, t.__name__, d, None if ours._CHOICES.get(n) is None else list(ours._CHOICES[n]))
+            for n, t, d, _ in ours._SPEC]
     assert [r[0] for r in ref] == [m[0] for m in mine]                       # same flags, same order
     for r, m in zip(ref, mine):
         assert r == m, (r, m)
     # and the defaults our parser hands out when neither a file nor a flag sets them
     a, _ = ours.parse_config(["--config", os.devnull])
-    for n, kw in recorded[1:]:
-        assert getattr(a, n) == kw.get("default"), n
+    for n, _, default, _ in ref:
+        assert getattr(a, n) == default, n

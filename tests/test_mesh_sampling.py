@@ -3,8 +3,8 @@
 Pinned by the reference itself: `data/transform_matrices/for_demo/{A,D,U}.npy` are the output of the reference's
 `generate_transform_matrices(template, [1, 2, 1, 2, 1, 2, 1, 1])` (psbody + qslim), and this restatement must
 reproduce them -- adjacency and down-sampling matrices exactly, up-sampling matrices to fp32 rounding.  The
-fixtures and the template are read from the locally packed copy (cape_b200.pack_topology), like every other test.
-The synthetic-mesh tests need no licensed data."""
+fixtures and the template are read from tests/golden/smpl_topology.*.npz (cape_b200.pack_topology), like every other
+test.  The synthetic-mesh tests need none of the reference's data."""
 import heapq
 
 import numpy as np
